@@ -604,6 +604,8 @@ extern "C" int acp_hostsim_run(acp_engine* engine, const char* config_json, char
   const int delegation_depth = std::max(0, std::min(4, (int)cfg.get("delegation_depth").as_int(0)));
   const uint64_t seed = (uint64_t)cfg.get("seed").as_int(1);
   const bool lease = cfg.find("emulate_lease") ? cfg.get("emulate_lease").as_bool(true) : true;
+  // report status.output of every root Task (by index) in the result: what the Task's owner reads back
+  const bool return_outputs = cfg.get("return_outputs").as_bool(false);
   if (provider == "local" && !engine) return ACP_ERR_INVALID;
 
   // agent-level tool list (collectTools): synthetic MCP tools server__tool_i
@@ -773,6 +775,7 @@ extern "C" int acp_hostsim_run(acp_engine* engine, const char* config_json, char
     }
   }
   std::vector<double> task_ms;   // arrival -> terminal phase of every ROOT Task
+  std::vector<std::string> outputs(return_outputs ? (size_t)std::max(0, n_tasks) : 0);
   const auto t0 = std::chrono::steady_clock::now();
   // Runs one Task (root or delegated child) to a terminal phase on the calling worker: the Task controller's
   // reconciles, with the (out of scope) ToolCall controller emulated in between — plain tools "execute" at once
@@ -874,6 +877,7 @@ extern "C" int acp_hostsim_run(acp_engine* engine, const char* config_json, char
         std::lock_guard<std::mutex> lk(lat_mu);
         task_ms.push_back(total_ms);
         ++phases[t.Status.Phase];
+        if (return_outputs) outputs[(size_t)i] = t.Status.Output;
         if (t.Status.Phase == "Failed" && first_error.empty())
           first_error = name + ": " + (t.Status.Error.empty() ? t.Status.StatusDetail : t.Status.Error);
         uint64_t h = 1469598103934665603ull;
@@ -913,6 +917,11 @@ extern "C" int acp_hostsim_run(acp_engine* engine, const char* config_json, char
   for (auto& kv : phases) ph.set(kv.first, Json(kv.second));
   out.set("final_phases", ph);
   if (!first_error.empty()) out.set("first_error", Json(first_error));   // why the first Failed Task failed
+  if (return_outputs) {
+    Json arr = Json::array();
+    for (const std::string& o : outputs) arr.push(Json(o));
+    out.set("outputs", arr);
+  }
   char dbuf[32];
   snprintf(dbuf, sizeof dbuf, "%016llx", (unsigned long long)digest);
   out.set("digest", Json(std::string(dbuf)));

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the hot path of BASELINE.json: Task reconciles through `provider: local`.
 
-  python bench.py --gpus N --steps K --warmup W [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic Task CRs: BASELINE config 2 (the
 largest single-GPU configuration, the one nearest north_star's ">= 1000 concurrent Task CRs"):
@@ -32,6 +32,12 @@ a provider; it cannot be built here (Go, no toolchain), so the arm runs the C++ 
 the reference's fixture body) on all host cores, on rank 0 only.  That restatement lives in its own
 library, libacp_host.so (pure C++, not linked against the product): the reference arm never maps
 libacp_infer.so.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step handed back to the Tasks'
+owner, DIR/task_output_bytes.npy: float32 [tasks, width], row i = the UTF-8 bytes of Task i's status.output,
+padded with -1.  width = 5 * max_tokens (a synthetic token decodes to at most 5 bytes), so the shape does not
+depend on what was generated.  Step i always runs seed i + 1: the same arguments give the same inputs, and
+two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -45,6 +51,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only: the benchmark writes nothing into it
 
 WORKLOADS = {
     # BASELINE.json configs[2]: the largest single-GPU configuration (default since round 2)
@@ -107,6 +114,19 @@ def window_cfg(w: dict) -> dict:
 def window_desc(w: dict) -> str:
     return (f"windows log-uniform {w['prompt_min']}..{w['prompt_max']} tokens" if w.get("prompt_min")
             else f"windows of {w['prompt_tokens']} tokens")
+
+
+def dump_outputs(out_dir: str, outputs: list, max_tokens: int) -> None:
+    """status.output of every Task as UTF-8 byte rows (float32, -1 padding) in out_dir/task_output_bytes.npy"""
+    import numpy as np
+    rows = [o.encode() for o in outputs]
+    width = max([5 * max_tokens] + [len(r) for r in rows])
+    arr = np.full((len(rows), width), -1.0, dtype=np.float32)
+    for i, r in enumerate(rows):
+        arr[i, :len(r)] = np.frombuffer(r, dtype=np.uint8)
+    assert arr.nbytes <= 64 << 20, arr.shape
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "task_output_bytes.npy"), arr)
 
 
 class ClockSampler:
@@ -230,7 +250,13 @@ def main():
                     help="BASELINE.json config index (2 = default; 1 = 64 x 512; 3 = 70B TP=8, 4 = Mixtral EP=8: ONE process on an 8-GPU box, --gpus 1)")
     ap.add_argument("--max-tokens-per-step", type=int, default=4096, help="engine knob: token rows per prefill step (4096 measured 1.3 %% faster than 8192)")
     ap.add_argument("--tp", type=int, default=0, help="dev only: override the tensor-parallel degree of --config 3")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the Task outputs of the last timed step to DIR/task_output_bytes.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the outputs of --impl ours")
     WORKLOAD = dict(WORKLOADS[args.config])
     if args.config in (3, 4):
         if args.model == WORKLOADS[1]["model"]:
@@ -318,7 +344,7 @@ def main():
     t0 = time.perf_counter()
     reconciles, p50s, phases, task_p50, task_p99 = 0, [], {}, [], []
     for i in range(args.steps):
-        r = host.hostsim_run(dict(sim, seed=i + 1), eng)
+        r = host.hostsim_run(dict(sim, seed=i + 1, return_outputs=bool(args.dump_outputs) and i == args.steps - 1), eng)
         reconciles += r["reconciles"]
         p50s.append(r["step_ms_p50"])
         task_p50.append(r.get("task_ms_p50"))
@@ -334,6 +360,8 @@ def main():
     wall = time.perf_counter() - t0
     clocks = sampler.stop() if sampler else None
     s1 = eng.stats()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r["outputs"], max_new)
     # extra key: BASELINE config 1 (64 Tasks x 512-token windows) on the same engine, outside the timed region
     config1 = None
     if args.config == 2 and rank == 0:

@@ -36,6 +36,25 @@ def test_reference_arm_never_maps_the_product_library():
     assert out.returncode == 0, out.stderr[-2000:]
 
 
+def test_dump_outputs_writes_fixed_width_byte_rows(tmp_path):
+    code = ("import runpy, sys\n"
+            "runpy.run_path(%r)['dump_outputs'](sys.argv[1], ['test', '', 'caf\\u00e9 ' * 3], 2)\n" % os.path.join(ROOT, "bench.py"))
+    out = subprocess.run([sys.executable, "-c", code, str(tmp_path / "d")], capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    import numpy as np
+    a = np.load(tmp_path / "d" / "task_output_bytes.npy")
+    assert a.dtype == np.float32 and a.shape == (3, 18)         # the third output is longer than 5 * max_tokens
+    assert a[0, :4].tolist() == list(b"test") and (a[0, 4:] == -1).all() and (a[1] == -1).all()
+    assert bytes(a[2].astype(np.uint8)) == "café café café ".encode()
+
+
+def test_steps_and_dump_arguments_are_checked():
+    for args in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "x"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True,
+                             timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and "error:" in out.stderr, (args, out.stderr[-500:])
+
+
 def test_reference_arm_follows_the_config_flag():
     j = _line("--impl", "reference", "--config", "3", "--steps", "1", "--warmup", "0")
     assert j["impl"] == "reference" and "256 concurrent Task CRs" in j["config"]["workload"]

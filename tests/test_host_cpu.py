@@ -238,7 +238,10 @@ def test_config0_plumbing_over_stub_server():
         assert st["phase"] == "FinalAnswer" and st["output"] == "test" and len(st["contextWindow"]) == 3
         r = host.hostsim_run({"tasks": 200, "workers": 4, "provider": "openai", "model": "gpt-4o", "baseURL": srv.base_url})
         assert r["reconciles"] == 200 and r["final_phases"] == {"FinalAnswer": 200}
-        assert r["store_writes"] >= 4 * 200 and r["reconciles_per_s"] > 0
+        assert r["store_writes"] >= 4 * 200 and r["reconciles_per_s"] > 0 and "outputs" not in r
+        r = host.hostsim_run({"tasks": 20, "workers": 4, "provider": "openai", "model": "gpt-4o", "baseURL": srv.base_url,
+                              "return_outputs": True})
+        assert r["outputs"] == ["test"] * 20
     tool_body = G["G8_wire_fixtures"]["tool_body"]["body"]
     with host.StubServer(tool_body) as srv:
         out = host.task_step({"op": "sendLLMRequest", "task": _task(), "tools": B.convert_mcp_tools([{"name": "fetch"}], "fetch"),
